@@ -20,6 +20,10 @@ graphs of the named architectures + seeded random weights (no checkpoints offlin
 Other workloads (`--workload`): sdxl_unet_w8 (SDXL 1024x1024, uint8 weights; N=2 = the CFG cond/uncond pair), sdxl_turbo_w8
 (512x512, one sample per GPU), vae_decoder_fp16, clip_text_fp32, sd15_pipeline (text encoder + 20 CFG steps + VAE decoder),
 tinyllama_decode (seq 2048).  `--all-configs FILE` runs them all and writes one line each.
+
+`--dump-outputs DIR` writes what the value arm computed in its last timed step -- every output tensor a caller of that
+path receives -- as DIR/<tensor>.npy (float32, float64 for int64 outputs; sd15_pipeline: DIR/<workload>.<tensor>.npy), at
+most 64 MB in all.  Inputs and weights are seeded, so two builds run on the same arguments can be compared output for output.
 """
 import argparse
 import ctypes
@@ -69,6 +73,7 @@ SHM = "/dev/shm" if os.path.isdir("/dev/shm") and os.access("/dev/shm", os.W_OK)
 REF_CACHE = os.path.join(SHM, "osb200_ref_cache")
 
 FP16 = ("use_fp16_arithmetic", "fuse_ops_in_attention")
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 # =====================================================================================================================
@@ -550,8 +555,31 @@ def run_reference(args):
 # =====================================================================================================================
 # the B200 arm
 # =====================================================================================================================
-def measure(w: Workload, args, dist, clocks=None):
-    """value / e2e / roofline / parity for one single-model workload; returns the JSON line (rank 0) or None."""
+def value_outputs(m):
+    """Every output tensor of the last run of `m`, as a caller of Model::run receives it."""
+    out = {}
+    for n in m.get_all_tensor_names():
+        t = m.get_tensor(n)
+        out[n] = m.get_tensor_i64(n) if t is None else t
+    return out
+
+
+def write_outputs(d, outputs):
+    """DIR/<name>.npy for every output, float32 (float64 for int64 / float64 tensors); an output larger than its share of
+    DUMP_LIMIT_BYTES is replaced by a fixed, seeded sample of its elements."""
+    os.makedirs(d, exist_ok=True)
+    share = DUMP_LIMIT_BYTES // max(len(outputs), 1)
+    for name, a in outputs.items():
+        a = np.asarray(a)
+        a = a.astype(np.float64 if a.dtype in (np.int64, np.float64) else np.float32)
+        if a.nbytes > share:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False))]
+        np.save(os.path.join(d, name + ".npy"), a)
+
+
+def measure(w: Workload, args, dist, clocks=None, outputs=None):
+    """value / e2e / roofline / parity for one single-model workload; returns the JSON line (rank 0) or None.
+    `outputs` (a dict): filled with what the value arm computed in its last timed step."""
     d, meta = ensure_model(w)
     dist_barrier(dist)
     inputs = w.inputs(RANK)   # rank r = sample r (seed + rank, src/sd.cpp:2671)
@@ -594,6 +622,11 @@ def measure(w: Workload, args, dist, clocks=None):
     gpu_ms = dist_max(dist, gpu_ms)
     ms_per_step = gpu_ms / args.steps
     value = WORLD * 1000.0 / ms_per_step
+    if outputs is not None:
+        if graph_ok:
+            # graph replays leave their outputs on the device: one more replay of the same graph on the same inputs returns them
+            step_api(mv, later, None)
+        outputs.update(value_outputs(mv))
 
     # ---------------- supplementary: host inputs / outputs through the C ABI every step, weights resident ----------------
     e2e_resident = None
@@ -738,7 +771,7 @@ def measure(w: Workload, args, dist, clocks=None):
     return line if RANK == 0 else None
 
 
-def run_pipeline(args, dist):
+def run_pipeline(args, dist, outputs=None):
     """BASELINE config[1]: text encoder (cond + uncond) + 20 sampler steps x 2 UNet runs (CFG) + VAE decoder = one 512x512 image.
     Each model is measured on its own (value / e2e as in `measure`); the image time is the sum over its calls."""
     parts = [("clip_text_fp32", 2), ("sd15_unet_fp16", 40), ("vae_decoder_fp16", 1)]
@@ -746,7 +779,10 @@ def run_pipeline(args, dist):
     lines, t_val, t_e2e, launches, h2d, d2h = {}, 0.0, 0.0, 0, 0, 0
     a2 = argparse.Namespace(**vars(args)); a2.no_cpu_baseline = True
     for name, calls in parts:
-        ln = measure(make_workload(name), a2, dist, clocks=ClockSampler())
+        part = None if outputs is None else {}
+        ln = measure(make_workload(name), a2, dist, clocks=ClockSampler(), outputs=part)
+        if part:
+            outputs.update({f"{name}.{k}": v for k, v in part.items()})
         if RANK == 0:
             lines[name] = ln
             t_val += calls * ln["ms_per_step"]; t_e2e += calls * ln["e2e"]["ms_per_step"]
@@ -776,7 +812,10 @@ def main():
     ap.add_argument("--workload", default="sd15_unet_fp16", choices=WORKLOADS)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--all-configs", default=None, help="run every BASELINE workload and append one JSON line each to this file")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.all_configs or args.impl == "reference"):
+        ap.error("--dump-outputs dumps the B200 path of one workload: it does not combine with --all-configs or --impl reference")
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
 
     if args.impl == "reference":
@@ -800,8 +839,11 @@ def main():
                 if name == "sd15_unet_fp16":
                     emit_line(line)
     else:
-        line = run_pipeline(args, dist) if args.workload == "sd15_pipeline" else measure(make_workload(args.workload), args, dist)
+        outputs = {} if args.dump_outputs else None
+        line = run_pipeline(args, dist, outputs) if args.workload == "sd15_pipeline" else measure(make_workload(args.workload), args, dist, outputs=outputs)
         if RANK == 0:
+            if outputs is not None:
+                write_outputs(args.dump_outputs, outputs)
             emit_line(line)
     if dist is not None:
         dist.destroy_process_group()

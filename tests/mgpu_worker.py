@@ -1,7 +1,7 @@
 """Worker of tests/test_multi_gpu.py: one process per GPU (torchrun), NCCL weight distribution through the engine's WeightStreamer.
 Every rank runs ITS OWN sample (seed = rank) on the tiny fp16 UNet with all weights streamed through the HBM ring -- sharded upload
 (1/N over this rank's PCIe link + ncclAllGather) by default, root upload + ncclBroadcast with OSB_SHARDED_H2D=0 -- and compares the
-result with the reference's CPU path (oracle/_ref) computed by the same rank.  Prints one MGPU_OK / MGPU_FAIL line per rank."""
+result with the reference's output for that sample (tests/golden/unet_tiny16_fp16_seed<rank>.npz).  Prints one MGPU_OK / MGPU_FAIL line per rank."""
 import ctypes
 import os
 import sys
@@ -19,7 +19,7 @@ import torch.distributed as dist  # noqa: E402
 from onnxstream_b200 import emit  # noqa: E402
 from onnxstream_b200.model import Model, ENGINE_LIB  # noqa: E402
 
-ORACLE = os.path.join(ROOT, "oracle", "_ref", "liboracle_ref.so")
+GOLDEN = np.load(os.path.join(ROOT, "tests", "golden", f"unet_tiny16_fp16_seed{RANK}.npz"))
 torch.cuda.set_device(0)
 dist.init_process_group("nccl", device_id=torch.device("cuda", 0))
 d = sys.argv[1]
@@ -56,7 +56,8 @@ assert comm, "ncclCommInitRank failed"
 probe.close()
 got, m = run(ENGINE_LIB, comm, runs=3)          # 3 runs: ring wrap-around and slot reuse across runs
 st = m.stats()
-ref, _ = run(ORACLE)
+assert all(np.array_equal(GOLDEN["in_" + k], v) for k, v in inputs.items()), "inputs differ from the stored case"
+ref = GOLDEN["output"]
 alone, _ = run(ENGINE_LIB, None)                # the same engine without NCCL: every byte over this rank's own link
 err = float(np.abs(got - ref).max()) / max(float(np.abs(ref).max()), 1e-9)
 self_err = float(np.abs(got - alone).max()) / max(float(np.abs(alone).max()), 1e-9)

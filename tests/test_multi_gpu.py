@@ -1,5 +1,5 @@
 """2-GPU parity (skips with < 2 GPUs): the NCCL weight-distribution paths of the WeightStreamer, checked on EVERY rank against the
-reference's CPU path -- rank 0 is the root that never receives data, so rank 1's output is the one that proves the collective."""
+reference's output (stored under tests/golden/) -- rank 0 is the root that never receives data, so rank 1's output is the one that proves the collective."""
 import os
 import subprocess
 import sys
@@ -23,7 +23,7 @@ def _ngpus():
 
 @pytest.mark.skipif(_ngpus() < 2, reason="needs 2 GPUs")
 @pytest.mark.parametrize("sharded", ["1", "0"])
-def test_two_ranks_match_reference(oracle_lib, sharded):
+def test_two_ranks_match_reference(sharded):
     with tempfile.TemporaryDirectory(prefix="osb200_mgpu_") as tmp:
         d = tmp + "/"
         emit.emit_unet(d, emit.UNetConfig.tiny(16), "float16", seed=0)
